@@ -7,7 +7,7 @@ plus the fused-kernel HBM GB/s against the measured roofline.
 A "step" is one Code2Vec.forward (fused gather+encode+attention kernel, per-bag finalize,
 label logits, argmax) over one batch of 1024 synthetic bags of 200 contexts.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W]            # our arm
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]    # our arm
     python bench.py --impl reference [...]                          # the reference's CPU path
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
@@ -170,6 +170,30 @@ def bench_config(w, args):
                   f"{nb} distinct batches ({nb * w['B'] * w['L'] * 24 / 1e6:.0f} MB of indices) cycled"}
 
 
+DUMP_BYTES = 64 << 20         # at most this much is written by --dump-outputs
+
+
+def dump_outputs(d, tensors):
+    """--dump-outputs: every result of the timed path's last step as <d>/<name>.npy, floating point as float32 and integers
+    as float64 (exact below 2**53).  If together they exceed DUMP_BYTES, the largest keeps a fixed, seeded sample of its
+    rows, whose indices go to <d>/<name>_rows.npy: two builds run with the same arguments write the same entries."""
+    import numpy as np
+    arrays = {k: t.detach().cpu().numpy() for k, t in tensors.items()}
+    arrays = {k: a.astype(np.float32 if a.dtype.kind == "f" else np.float64) for k, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        big = max(arrays, key=lambda k: arrays[k].nbytes)
+        a = arrays[big]
+        row_bytes = a.nbytes // a.shape[0] + 8
+        n = max(1, (DUMP_BYTES - (total - a.nbytes)) // row_bytes)
+        rows = np.sort(np.random.default_rng(0).choice(a.shape[0], size=n, replace=False))
+        arrays[big] = a[rows]
+        arrays[big + "_rows"] = rows.astype(np.float64)
+    os.makedirs(d, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(d, k + ".npy"), a)
+
+
 def find_reference_module():
     """The UNMODIFIED reference `model.model.Code2Vec` if it can be imported on this box: baseline/_ref first, then
     /root/reference (BASELINE.md section 3.1).  The reference has neither setup.py nor pyproject.toml, so the offline pip
@@ -257,7 +281,7 @@ def run_reference(args, w):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=2000)
+    ap.add_argument("--steps", type=int, help="timed steps (default: 2000 on the GPU, 20 for --impl reference)")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="cfg2", choices=sorted(WORKLOADS))
@@ -273,12 +297,18 @@ def main():
     ap.add_argument("--no-gpu-eager", action="store_true", help="skip the ATen/cuBLAS eager comparator on this GPU")
     ap.add_argument("--transport", default="auto", choices=["auto", "nvls", "p2p", "nccl"],
                     help="gradient reduction of the training leg (ShardedFlatAdam)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step (rank 0) to DIR/<name>.npy, at most 64 MB in all")
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 20 if args.impl == "reference" else 2000
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes what the CUDA path computed; --impl reference has no such outputs")
     w = dict(WORKLOADS[args.workload]); w["name"] = args.workload
 
     if args.impl == "reference":
-        if args.steps == 2000:
-            args.steps = 20
         return run_reference(args, w)
 
     # The measured loops are CUDA-API-bound on ONE host thread; a 128-thread OpenMP/ATen pool in the same
@@ -361,14 +391,12 @@ def main():
         parity["ok"] = max(parity["max_abs_err"].values()) <= 1e-4
 
     # ---- device-resident throughput ("value") --------------------------------------------------
-    # The driver runs --steps 20: one pass of K steps lasts ~2 ms, too short for clocks sampling or kernel statistics.
-    # The K-step pass (barrier + synchronize on both sides, CUDA events around exactly K steps) is therefore REPEATED
-    # until >= MIN_REGION_S of GPU time has been measured; the reported ms_per_step is the MEDIAN pass.
-    MIN_REGION_S = 0.6
+    # --warmup steps, then the timed region: exactly --steps steps (batches W .. W+K-1 of the pool, so the same arguments
+    # give the same inputs), bracketed by barrier + synchronize and timed with CUDA events on the launch stream.
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    for i in range(max(args.warmup, 3)):
+    for i in range(args.warmup):
         step(i)
     barrier()
 
@@ -381,31 +409,34 @@ def main():
         barrier()
         return ev0.elapsed_time(ev1)
 
-    probe = timed_pass(args.warmup)                            # untimed: sizes the repetition count
-    tp = torch.tensor([probe], dtype=torch.float64, device=dev)
-    if dist is not None:
-        dist.all_reduce(tp, op=dist.ReduceOp.MAX)
-    reps = int(min(2000, max(3, -(-MIN_REGION_S * 1e3 // max(float(tp.item()), 1e-3)))))
     sampler.mark_begin()
-    lib.c2v_profile_enable(8)              # CUDA events around the dominant kernel on every 8th step of the timed loop
     l0 = lib.c2v_launch_count()
     t_wall0 = time.perf_counter()
-    pass_ms = [timed_pass(args.warmup + (r + 1) * args.steps) for r in range(reps)]
+    pass_ms = timed_pass(args.warmup)
     timed_region_s = time.perf_counter() - t_wall0
     sampler.mark_end()
-    launches = (lib.c2v_launch_count() - l0) / reps           # per K-step pass
+    launches = lib.c2v_launch_count() - l0
+    clocks = sampler.stop() if rank == 0 else None
+    t = torch.tensor([pass_ms], dtype=torch.float64, device=dev)
+    lt = torch.tensor([float(launches)], dtype=torch.float64, device=dev)
+    if dist is not None:
+        dist.all_reduce(t, op=dist.ReduceOp.MAX); dist.all_reduce(lt, op=dist.ReduceOp.SUM)   # the slowest rank
+    ms_max = float(t.item())
+    value = world * B * L * args.steps / (ms_max * 1e-3)
+    if rank == 0 and args.dump_outputs:
+        # the last timed step's results, before the legs below reuse the buffers (.gitignore lists these file names)
+        dump_outputs(args.dump_outputs, {"outputs": out, "code_vector": cv, "attention": att, "predicted_label": am,
+                                         "predicted_score": mx})
+
+    # ---- roofline of the dominant kernel (this rank) -----------------------------------------------
+    # CUDA events around every 8th launch of the kernel, in untimed passes of K steps after the timed one (>= 0.6 s of GPU
+    # time: hundreds of samples), so that no extra event sits inside the timed region
+    lib.c2v_profile_enable(8)
+    for r in range(int(min(2000, max(1, -(-600.0 // max(ms_max, 1e-3)))))):     # ms_max: the same count on every rank
+        timed_pass(args.warmup + (r + 1) * args.steps)
     kms, kcnt = ctypes.c_double(0), ctypes.c_int64(0)
     lib.c2v_profile_read(ctypes.byref(kms), ctypes.byref(kcnt))
     lib.c2v_profile_enable(0)
-    clocks = sampler.stop() if rank == 0 else None
-    t = torch.tensor(pass_ms, dtype=torch.float64, device=dev)
-    lt = torch.tensor([float(launches)], dtype=torch.float64, device=dev)
-    if dist is not None:
-        dist.all_reduce(t, op=dist.ReduceOp.MAX); dist.all_reduce(lt, op=dist.ReduceOp.SUM)   # per pass: max over ranks
-    ms_max = float(t.median().item())
-    value = world * B * L * args.steps / (ms_max * 1e-3)
-
-    # ---- roofline of the dominant kernel (this rank) -----------------------------------------------
     peak, peak_src = measured_peaks()
     k_ms = kms.value / max(1, kcnt.value)
     alg_bytes = bytes_per_ctx(w) * B * L
@@ -425,7 +456,7 @@ def main():
                 "achieved": achieved, "peak": peak, "unit": "GB/s", "frac": achieved / peak, "traffic": traffic,
                 "kernel_ms": k_ms, "kernel_samples": int(kcnt.value), "algorithmic_bytes_per_launch": alg_bytes,
                 "peak_source": peak_src, "ctx_per_s_kernel_only": B * L / (k_ms * 1e-3) if k_ms > 0 else 0.0,
-                "how": "CUDA events on the launch stream around every 8th launch of the kernel inside the timed passes "
+                "how": "CUDA events on the launch stream around every 8th launch of the kernel, in untimed passes after the timed one "
                        "(launch + prologue inside the interval, no dependent-launch overlap for the bracketed launch)"}
 
     # ---- the same kernel launched back to back (no bracketing events between launches, dependent-launch overlap intact):
@@ -524,20 +555,16 @@ def main():
             prev = cur
             if tw.item() > 0:
                 break
-        te = torch.tensor([prev], dtype=torch.float64, device=dev)
+        te = torch.tensor([host_pass()], dtype=torch.float64, device=dev)   # the timed pass: exactly --steps steps
         if dist is not None:
-            dist.all_reduce(te, op=dist.ReduceOp.MAX)
-        e_reps = int(min(400, max(3, -(-MIN_REGION_S // max(float(te.item()), 1e-6)))))
-        te = torch.tensor([host_pass() for _ in range(e_reps)], dtype=torch.float64, device=dev)
-        if dist is not None:
-            dist.all_reduce(te, op=dist.ReduceOp.MAX)           # per pass: the slowest rank
-        dt = float(te.median().item())
+            dist.all_reduce(te, op=dist.ReduceOp.MAX)           # the slowest rank
+        dt = float(te.item())
         lib.c2v_session_destroy(sess)
         e2e = {"value": world * B * L * args.steps / dt, "unit": "ctx/s",
                "h2d_bytes_per_step": 3 * B * L * 8, "d2h_bytes_per_step": B * H * 4 + B * L * 4 + B * 8 + B * 4 + 8,
                "api": "c2v_forward_host_async (4 batches in flight on upload / compute / download streams; pinned host int64 indices in, code_vector + "
                       "attention + argmax/score out; the [B, C] logits stay on the device: this is the predict surface of main.py:282-285)",
-               "ms_per_step": dt / args.steps * 1e3, "passes": e_reps, "warmup_passes": n_warm, "cpu_binding": bound}
+               "ms_per_step": dt / args.steps * 1e3, "warmup_passes": n_warm, "cpu_binding": bound}
 
     # ---- training step (reported beside the metric, not the metric): main.py:171-175 on this rank's shard; the gradient
     #      reduction over the ranks is fused into the optimizer kernel (ShardedFlatAdam, NVLS) -- no NCCL call in the step
@@ -611,10 +638,9 @@ def main():
             "metric": "path-contexts/sec", "value": value, "unit": "ctx/s", "n_gpus": world, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": ms_max / args.steps, "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "f32", "data": "synthetic", "config": cfg,
-            "timing": {"passes": reps, "pass_ms_median": ms_max, "pass_ms_min": float(t.min().item()),
-                       "pass_ms_max": float(t.max().item()), "timed_region_s": timed_region_s, "algo": args.algo,
-                       "how": f"{reps} passes of exactly {args.steps} steps, each bracketed by barrier + synchronize and timed "
-                              "with CUDA events on the launch stream; max over ranks per pass, median over passes"},
+            "timing": {"pass_ms": ms_max, "timed_region_s": timed_region_s, "algo": args.algo,
+                       "how": f"one pass of exactly {args.steps} steps after {args.warmup} warm-up steps, bracketed by barrier + "
+                              "synchronize and timed with CUDA events on the launch stream; max over ranks"},
             "roofline": roofline, "cpu_baseline": cpu, "gpu_eager_baseline": gpu_eager, "e2e": e2e, "train": train,
             "clocks": clocks, "gpu_launches": int(round(lt.item())), "parity": parity,
         }))
@@ -649,6 +675,7 @@ if __name__ == "__main__":
     # stdout carries the ONE JSON line and nothing else: libraries that write to file descriptor 1 during the run (NCCL's
     # "NCCL version ..." banner at communicator creation) are sent to stderr; print() goes to the real stdout at the end.
     import io
+    sys.dont_write_bytecode = True      # the tree may be read-only: the run writes nothing into it
     sys.stdout.flush()
     _real_stdout = os.dup(1)
     os.dup2(2, 1)

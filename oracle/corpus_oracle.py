@@ -9,7 +9,7 @@ TEST INFRASTRUCTURE ONLY: the checker of `c2v_corpus_parse_*` / `c2v_write_code_
   synthetic_corpus  seeded generator of a small corpus.txt / *_idxs.txt triple with the edge cases the format allows
 
 Pinned to the reference by tests/golden/reader_synth.npz (the reference's own DatasetReader run on synthetic_corpus(seed)
-by oracle/gen_golden.py) and tests/golden/reader_real.json (checksums of its output on dataset/corpus.txt).
+by oracle/gen_golden_io.py).
 """
 import re
 

@@ -25,6 +25,8 @@ sys.path.insert(0, REF)
 from model.model import Code2Vec  # noqa: E402  (the reference, unmodified)
 
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "tests", "golden")
+sys.path.insert(0, os.path.join(OUT, ".."))
+from conftest import params_sha256  # noqa: E402  (the digest tests/conftest.py checks)
 os.makedirs(OUT, exist_ok=True)
 
 
@@ -58,7 +60,9 @@ def make_inputs(gen, B, L, T, P, C, pad="suffix", holes=False, allpad_rows=()):
     return starts, paths, ends, label
 
 
-def dump(name, opt, model, starts, paths, ends, label, grads=False, scale=None):
+def dump(name, opt, model, starts, paths, ends, label, grads=False, scale=None, param_seed=None):
+    """param_seed: the torch.manual_seed the model was built under (plain head, unscaled).  A record that would exceed
+    1 MB then stores the seed and a digest of the parameters instead of the parameters (tests/conftest.py rebuilds them)."""
     model.eval()
     if scale:
         with torch.no_grad():
@@ -91,6 +95,12 @@ def dump(name, opt, model, starts, paths, ends, label, grads=False, scale=None):
     rec["attention"] = att.detach().numpy()
     path = os.path.join(OUT, name + ".npz")
     np.savez_compressed(path, **rec)
+    if param_seed is not None and os.path.getsize(path) > 1_000_000:
+        params = {k[6:]: v for k, v in rec.items() if k.startswith("param.")}
+        rec = {k: v for k, v in rec.items() if not k.startswith("param.")}
+        rec["param_seed"] = np.int64(param_seed)
+        rec["param_sha256"] = np.str_(params_sha256(params))
+        np.savez_compressed(path, **rec)
     print(f"{name:22s} B={starts.shape[0]:3d} L={starts.shape[1]:3d} -> {os.path.getsize(path)/1024:.0f} KiB")
 
 
@@ -121,7 +131,8 @@ def seeded(name, seed, B, L, T, P, C, Et, Ep, H, grads=False, scale=None, angula
     m = Code2Vec(opt)
     gen = torch.Generator().manual_seed(seed + 1000)
     starts, paths, ends, label = make_inputs(gen, B, L, T, P, C, **kw)
-    dump(name, opt, m, starts, paths, ends, label, grads=grads, scale=scale)
+    dump(name, opt, m, starts, paths, ends, label, grads=grads, scale=scale,
+         param_seed=seed if scale is None and not angular else None)
 
 
 def real_batch():

@@ -5,14 +5,12 @@ by running the UNMODIFIED reference (imported from /root/reference, never copied
     PYTHONDONTWRITEBYTECODE=1 python oracle/gen_golden_io.py
 
   tests/golden/reader_synth.npz   reference DatasetReader on oracle.corpus_oracle.synthetic_corpus(seed) (seeds 1, 2)
-  tests/golden/reader_real.json   checksums of the reference DatasetReader's output on dataset/corpus.txt
   tests/golden/builder_vars.npz   reference DatasetBuilder.build_data, infer_variable branch (dataset_builder.py:152-204)
   tests/golden/writer.npz         reference write_code_vectors (main.py:393-423) output for fixed vectors
   tests/golden/unaligned.npz, grad_unaligned.npz   forward / gradient goldens with embed / encode sizes not divisible by 4
   tests/golden/grad_wide.npz, grad_e200.npz        gradient goldens with embed / encode sizes above 128
 """
 import ast
-import hashlib
 import json
 import os
 import random
@@ -33,10 +31,6 @@ from model.dataset_builder import DatasetBuilder  # noqa: E402
 from model.dataset_reader import DatasetReader    # noqa: E402
 
 REF, OUT = gg.REF, gg.OUT
-
-
-def _sha(a):
-    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
 
 
 def _reader_record(reader):
@@ -81,21 +75,6 @@ def reader_synth():
                 rec[f"s{seed}_{tag}_contexts"] = ctx
     np.savez_compressed(os.path.join(OUT, "reader_synth.npz"), **rec)
     print("reader_synth:", len(rec), "arrays")
-
-
-def reader_real():
-    r = DatasetReader(f"{REF}/dataset/corpus.txt", f"{REF}/dataset/path_idxs.txt", f"{REF}/dataset/terminal_idxs.txt",
-                      infer_method=True, infer_variable=True, shuffle_variable_indexes=False)
-    meta, off, ctx = _reader_record(r)
-    out = {"n_items": len(r.items), "n_contexts": int(off[-1]), "ids_sha": _sha(np.asarray(meta["ids"], np.int64)),
-           "offsets_sha": _sha(off), "contexts_sha": _sha(ctx.astype(np.int32)),
-           "label_names_sha": hashlib.sha256("\n".join(meta["label_names"]).encode()).hexdigest(),
-           "n_labels": len(meta["label_names"]), "n_variable_indexes": len(meta["variable_indexes"]),
-           "aliases_sha": hashlib.sha256(json.dumps(meta["aliases"], ensure_ascii=False).encode()).hexdigest(),
-           "terminal_count": meta["terminal_count"], "path_count": meta["path_count"]}
-    with open(os.path.join(OUT, "reader_real.json"), "w") as f:
-        json.dump(out, f, indent=1)
-    print("reader_real:", out["n_items"], "items", out["n_contexts"], "contexts", out["n_labels"], "labels")
 
 
 def builder_vars():
@@ -178,7 +157,6 @@ def writer():
 
 if __name__ == "__main__":
     reader_synth()
-    reader_real()
     builder_vars()
     writer()
     gg.seeded("unaligned", 21, 6, 9, 23, 17, 5, 10, 7, 9, holes=True, allpad_rows=(3,))

@@ -1,4 +1,5 @@
 import glob
+import hashlib
 import os
 import sys
 
@@ -23,6 +24,34 @@ def golden_names(prefix=None, exclude_prefix=("init_", "builder_", "reader_", "w
     return names
 
 
+def params_sha256(params):
+    """Digest of a state dict's arrays (fp32 bytes, in order): pins the parameters a golden file stores by seed."""
+    h = hashlib.sha256()
+    for k, v in params.items():
+        h.update(k.encode())
+        h.update(np.ascontiguousarray(v, dtype=np.float32).tobytes())
+    return h.hexdigest()
+
+
+def reference_init_params(opt, seed):
+    """The reference's initial weights of a plain-head model under torch.manual_seed(seed): its modules in its order
+    (model.py:21-42), output bias zero-filled.  Golden files whose parameters are too large to store keep only the seed."""
+    import torch
+    import torch.nn as nn
+    torch.manual_seed(seed)
+    te = nn.Embedding(opt["T"], opt["Et"])
+    pe = nn.Embedding(opt["P"], opt["Ep"])
+    lin = nn.Linear(2 * opt["Et"] + opt["Ep"], opt["H"], bias=False)
+    ln = nn.LayerNorm(opt["H"])
+    att = nn.init.xavier_normal_(torch.zeros(opt["H"], 1)).view(-1)
+    out = nn.Linear(opt["H"], opt["C"], bias=True)
+    out.bias.data.fill_(0.0)
+    p = {"attention_parameter": att, "terminal_embedding.weight": te.weight, "path_embedding.weight": pe.weight,
+         "input_linear.weight": lin.weight, "input_layer_norm.weight": ln.weight, "input_layer_norm.bias": ln.bias,
+         "output_linear.weight": out.weight, "output_linear.bias": out.bias}
+    return {k: v.detach().numpy().copy() for k, v in p.items()}
+
+
 def load_golden(name):
     """-> dict(opt=..., params={state_dict key: array}, grads={...}, inputs..., outputs...)"""
     z = np.load(os.path.join(GOLDEN, name + ".npz"))
@@ -34,8 +63,12 @@ def load_golden(name):
             rec["params"][k[6:]] = z[k]
         elif k.startswith("grad."):
             rec["grads"][k[5:]] = z[k]
-        else:
+        elif k not in ("param_seed", "param_sha256"):
             rec[k] = z[k]
+    if "param_seed" in z.files:
+        rec["params"] = reference_init_params(rec["opt"], int(z["param_seed"]))
+        assert params_sha256(rec["params"]) == str(z["param_sha256"]), \
+            f"{name}: torch.manual_seed({int(z['param_seed'])}) no longer yields the reference's initial weights"
     return rec
 
 
