@@ -7,7 +7,7 @@ import ctypes
 import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("C2V_LIB", os.path.join(_HERE, "libc2v_b200.so"))   # C2V_LIB: variant builds (experiments)
+LIB_PATH = os.environ.get("C2V_LIB", os.path.join(_HERE, "libc2v_b200.so"))   # C2V_LIB: variant builds (scripts/sanitize.sh)
 
 C2V_OK, C2V_EINVAL, C2V_ECUDA, C2V_EWORKSPACE, C2V_EINDEX, C2V_EUNSUPPORTED = 0, -1, -2, -3, -4, -5
 ALGO_AUTO, ALGO_FFMA, ALGO_TCGEN05 = 0, 1, 2

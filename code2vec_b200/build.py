@@ -8,14 +8,10 @@ import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
-OUT = os.environ.get("C2V_LIB_OUT", os.path.join(HERE, "libc2v_b200.so"))   # experiments: variant builds
+OUT = os.environ.get("C2V_LIB_OUT", os.path.join(HERE, "libc2v_b200.so"))   # variant builds (scripts/sanitize.sh)
 EXTRA = os.environ.get("C2V_NVCC_EXTRA", "").split()
-# c2v_encode_tma.cu / c2v_encode_cpa.cu (and the K1b kernel inside c2v_encode_tcgen05.cu) are superseded encode variants
-# kept for A/B timing: compiled only with C2V_NVCC_EXTRA=-DC2V_EXPERIMENTS (then selected by C2V_ENCODE_KERNEL=tma|cpa|ldg)
-EXPERIMENT_SOURCES = ["c2v_encode_tma.cu", "c2v_encode_cpa.cu"] if "-DC2V_EXPERIMENTS" in os.environ.get("C2V_NVCC_EXTRA", "") else []
-SOURCES = ["c2v_api.cu", "c2v_session.cu", "c2v_encode_ffma.cu", "c2v_encode_tcgen05.cu", "c2v_encode_tm.cu", "c2v_label_tcgen05.cu", "c2v_label_backward_tc.cu", "c2v_head.cu",
-           "c2v_backward.cu", "c2v_backward_dw_tc.cu", "c2v_backward_dc_tc.cu", "c2v_batch.cu", "c2v_adam.cu", "c2v_corpus.cpp"] + \
-          EXPERIMENT_SOURCES
+SOURCES = ["c2v_api.cu", "c2v_session.cu", "c2v_encode_ffma.cu", "c2v_encode_tm.cu", "c2v_label_tcgen05.cu", "c2v_label_backward_tc.cu", "c2v_head.cu",
+           "c2v_backward.cu", "c2v_backward_dw_tc.cu", "c2v_backward_dc_tc.cu", "c2v_batch.cu", "c2v_adam.cu", "c2v_corpus.cpp"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
          "-Xcompiler", "-fPIC", "-Xcompiler", "-Wall", "--expt-relaxed-constexpr"]

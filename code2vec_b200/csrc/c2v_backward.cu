@@ -547,18 +547,19 @@ int launch_encode_backward(const c2v_dims *d, const c2v_params *p, const EncodeA
     float *w_t = reinterpret_cast<float *>(base + o); o += align_up((size_t)a.D * Hs * 4, 1024);
     unsigned *dx_absmax = reinterpret_cast<unsigned *>(base + o); o += 1024;
     void *dc_ws = base + o;
-    {
-        const char *dc_env0 = getenv("C2V_BACKWARD_DC"), *dw_env0 = getenv("C2V_BACKWARD_DW");
-        const bool split_ok = x_stash && (a.H & 3) == 0 && backward_dc_tc_ok(a) && backward_dw_tc_ok(a) &&
-                              !(dc_env0 && !strcmp(dc_env0, "ffma")) && !(dw_env0 && !strcmp(dw_env0, "ffma"));
-        if (phase == 2) {
-            if (!split_ok) return C2V_OK;                       // phase 1 already did everything
-            a.n_tiles = (int)((a.N + TM - 1) / TM);
-            return launch_backward_dc_tc(a, p->input_linear, dx, dx_absmax, dc_ws, g->terminal_embedding, g->path_embedding, st,
-                                         5, false);
-        }
-        if (phase == 1 && !split_ok) phase = 0;
+    // dC = dX . W and dW = dX^T . C run on the tensor cores when the shape allows.  C2V_BACKWARD=ffma keeps both on the
+    // CUDA cores: the reference the tensor-core tests compare against.
+    const char *impl = getenv("C2V_BACKWARD");
+    const bool ffma = impl && !strcmp(impl, "ffma");
+    const bool dc_tc = !ffma && backward_dc_tc_ok(a), dw_tc = !ffma && backward_dw_tc_ok(a);
+    const bool split_ok = x_stash && (a.H & 3) == 0 && dc_tc && dw_tc;
+    if (phase == 2) {
+        if (!split_ok) return C2V_OK;                           // phase 1 already did everything
+        a.n_tiles = (int)((a.N + TM - 1) / TM);
+        return launch_backward_dc_tc(a, p->input_linear, dx, dx_absmax, dc_ws, g->terminal_embedding, g->path_embedding, st,
+                                     5, false);
     }
+    if (phase == 1 && !split_ok) phase = 0;
     C2V_CUDA_OK(cudaMemsetAsync(dx_absmax, 0, 4, st));
     memset(&a.ws, 0, sizeof(a.ws));
     a.ws.w_t = w_t;
@@ -569,9 +570,6 @@ int launch_encode_backward(const c2v_dims *d, const c2v_params *p, const EncodeA
     if (rc != C2V_OK) return rc;
     BackwardArgs b;
     b.cv = cv; b.att = attention; b.d_cv = d_cv; b.d_att = d_att; b.sb = nullptr; b.x_stash = x_stash; b.dx_absmax = dx_absmax;
-    // dC = dX . W and dW = dX^T . C run on the tensor cores when the shape allows; C2V_BACKWARD_DC / _DW = ffma force CUDA cores
-    const char *dc_env = getenv("C2V_BACKWARD_DC");
-    const bool dc_tc = backward_dc_tc_ok(a) && !(dc_env && !strcmp(dc_env, "ffma"));
     b.skip_dc = dc_tc ? 1 : 0;
     b.W = p->input_linear; b.dx = dx;
     b.g_emb_t = g->terminal_embedding; b.g_emb_p = g->path_embedding;
@@ -607,32 +605,23 @@ int launch_encode_backward(const c2v_dims *d, const c2v_params *p, const EncodeA
         }
         rc = launch_backward_dc_tc(a, p->input_linear, dx, dx_absmax, dc_ws, g->terminal_embedding, g->path_embedding, st, 7, true);
         if (rc != C2V_OK) return rc;
-        const char *dw_env2 = getenv("C2V_BACKWARD_DW");
-        if (backward_dw_tc_ok(a) && !(dw_env2 && !strcmp(dw_env2, "ffma")))
-            return launch_backward_dw_tc(a, dx, dx_absmax, g->input_linear, st);
-        a.n_tiles = (int)((a.N + TM - 1) / TM);
-        goto dw_ffma;
-    }
-    {
-    auto kern = vec ? backward_rows_kernel<true> : backward_rows_kernel<false>;
-    C2V_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    int occ = 1;
-    C2V_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, THREADS, smem));
-    if (occ < 1) occ = 1;
-    int grid = a.n_tiles < sms * occ ? a.n_tiles : sms * occ;
-    kern<<<grid, THREADS, smem, st>>>(a, b, Hs);
-    C2V_LAUNCH_OK("backward_rows_kernel");
-    if (dc_tc) {
-        rc = launch_backward_dc_tc(a, p->input_linear, dx, dx_absmax, dc_ws, g->terminal_embedding, g->path_embedding, st, 7, true);
-        if (rc != C2V_OK) return rc;
+    } else {
+        auto kern = vec ? backward_rows_kernel<true> : backward_rows_kernel<false>;
+        C2V_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        int occ = 1;
+        C2V_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, THREADS, smem));
+        if (occ < 1) occ = 1;
+        int grid = a.n_tiles < sms * occ ? a.n_tiles : sms * occ;
+        kern<<<grid, THREADS, smem, st>>>(a, b, Hs);
+        C2V_LAUNCH_OK("backward_rows_kernel");
+        if (dc_tc) {
+            rc = launch_backward_dc_tc(a, p->input_linear, dx, dx_absmax, dc_ws, g->terminal_embedding, g->path_embedding, st, 7, true);
+            if (rc != C2V_OK) return rc;
+        }
     }
 
-    // dW = dX^T . C: tensor cores when the shape allows (c2v_backward_dw_tc.cu), C2V_BACKWARD_DW=ffma forces the CUDA cores
-    const char *dw_env = getenv("C2V_BACKWARD_DW");
-    if (backward_dw_tc_ok(a) && !(dw_env && !strcmp(dw_env, "ffma")))
-        return launch_backward_dw_tc(a, dx, dx_absmax, g->input_linear, st);
-    }
-dw_ffma:
+    // dW = dX^T . C
+    if (dw_tc) return launch_backward_dw_tc(a, dx, dx_absmax, g->input_linear, st);
     const int gx = (a.D + DW_T - 1) / DW_T, gy = (a.H + DW_T - 1) / DW_T;
     long long split = (8LL * sms) / (gx * gy);
     if (split < 1) split = 1;

@@ -38,21 +38,11 @@ extern long long g_launches;
 
 static inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
-// Timing experiments (skip a role's work to see what the others cost; results become wrong) exist only in builds
-// with -DC2V_EXPERIMENTS (C2V_NVCC_EXTRA=-DC2V_EXPERIMENTS python -m code2vec_b200.build); product builds compile them out.
-#ifdef C2V_EXPERIMENTS
-#define C2V_EXPT(flags, bit) (((flags) & (bit)) != 0)
-#else
-#define C2V_EXPT(flags, bit) false
-#endif
-
 #ifdef __CUDACC__
 // Programmatic dependent launch: the kernel may start (prologue, block scheduling) while the previous kernel of the
 // stream is still draining; it must execute griddepcontrol.wait (pdl_wait()) before touching anything the previous
-// kernel wrote.  C2V_NO_PDL=1 falls back to a plain launch (A/B timing).
-bool pdl_enabled();
-// per-call switch (thread local, set by the extern "C" entry points): the calls that feed autograd -- the stashing training
-// forward, or any call with C2V_FLAG_NO_PDL -- use plain stream-ordered launches
+// kernel wrote.  Per-call switch (thread local, set by the extern "C" entry points): the calls that feed autograd -- the
+// stashing training forward, or any call with C2V_FLAG_NO_PDL -- use plain stream-ordered launches.
 extern thread_local bool g_pdl_this_call;
 template <typename... KArgs, typename... Args>
 static inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args)
@@ -62,7 +52,7 @@ static inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 blo
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = (pdl_enabled() && g_pdl_this_call) ? 1 : 0;
+    cfg.attrs = attr; cfg.numAttrs = g_pdl_this_call ? 1 : 0;
     return cudaLaunchKernelEx(&cfg, kern, KArgs(args)...);
 }
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
@@ -76,7 +66,6 @@ struct EncodeWorkspace {
     float *prep_hdr;       // [0] 1/w_scale (tcgen05 path), [1] w_scale
     float *w_t;            // FFMA: W transposed, [D][Hs] fp32 (Hs = H rounded up to 4)
     uint16_t *w_hi;        // tcgen05: per k-block {hi, lo} fp16 tiles of W*scale, UMMA K-major SW128
-    uint16_t *w_lo;        //          (unused; the lo tile follows its hi tile inside w_hi)
     float *part_m;         // [slots] running max of each (tile, bag) segment
     float *part_s;         // [slots] sum of exp(z - m)
     float *part_v;         // [slots][H] sum of exp(z - m) * h
@@ -100,14 +89,11 @@ struct EncodeArgs {
     unsigned long long seed;
     float *attention;       // [N] raw masked scores z (finalize turns them into softmax weights)
     float *stash_x;         // optional [N, H]: x = c . W^T (model.py:54) of every row, kept for the backward
-    int flags;              // debug switches (bit 0: producer-side proxy fence in the tcgen05 kernel)
     EncodeWorkspace ws;
 };
 
-int launch_prepare_weights(const c2v_dims *d, const float *W, EncodeWorkspace &ws, bool tcgen05,
-                           cudaStream_t st);
 int launch_encode_ffma(const EncodeArgs &a, cudaStream_t st);
-int launch_encode_tcgen05(const EncodeArgs &a, cudaStream_t st);
+int launch_encode_tm(const EncodeArgs &a, cudaStream_t st);
 bool tcgen05_shape_ok(const c2v_dims *d);
 int launch_encode_finalize(const EncodeArgs &a, int B, float *code_vector, cudaStream_t st);
 

@@ -1,12 +1,22 @@
-// c2v_encode_tm.cu -- K1e: fused gather + encode + attention, activations operand in TENSOR MEMORY.
+// c2v_encode_tm.cu -- K1e: the fused gather + encode + attention kernel on the 5th-gen tensor cores (sm_100a), with
+// its shape check (tcgen05_shape_ok) and its weight preparation (split_w_kernel).
 //
-// Same numerics / epilogue as K1b-K1d (model.py:48-69 + 90-96; 3-pass fp16 split, c2v_encode_tcgen05.cu), but the
-// gathered-and-split A operand never goes back to shared memory: the converter warps write the fp16 hi/lo
-// halves straight into TMEM with tcgen05.st and the MMAs read A from TMEM (tcgen05.mma [d], [a_tmem], b_desc).
-// Why (profiles/README.md, K1d): K1d moved 224 KB through shared memory per k-block (cp.async 32 + LDS 32 +
-// STS 32 + W copy 32 + MMA operand reads 96) = ~60 us per cfg2 batch at 128 B/clk, and its two 32 KB raw stages
-// kept only 64 KB of gathers in flight per SM (loaders alone: 69 us).  Here the STS and the MMA's A reads are
-// gone (144 KB per k-block) and the 64 KB of smem they occupied became two more raw stages (128 KB in flight).
+// What it replaces: model.py:48-69 + get_attention (model.py:90-96) of the reference.
+//
+// Numerics.  The reference contraction x = c . W^T is fp32; plain TF32/BF16 miss the 1e-4 parity bar (SURVEY.md 8d).
+// Here both operands are split into fp16 hi + fp16 lo (a = a_hi + a_lo exactly to ~2^-22) and three kind::f16 MMAs
+// with fp32 accumulation are issued per k-step:  a_hi.w_hi + a_lo.w_hi + a_hi.w_lo  (the dropped a_lo.w_lo term is
+// 2^-22 relative).  W is pre-multiplied by a power of two so its lo part stays out of the fp16 subnormals; the
+// epilogue (c2v_tc_epilogue.cuh) folds the exact inverse into the LayerNorm scale.
+// Measured distance to the reference: ~5e-7 (tests/test_forward_parity_gpu.py).
+//
+// The gathered-and-split A operand lives in TENSOR MEMORY: the converter warps write the fp16 hi/lo halves straight
+// into TMEM with tcgen05.st and the MMAs read A from TMEM (tcgen05.mma [d], [a_tmem], b_desc).
+// Why (profiles/README.md): K1d, the earlier variant with A in shared memory, moved 224 KB through shared memory per
+// k-block (cp.async 32 + LDS 32 + STS 32 + W copy 32 + MMA operand reads 96) = ~60 us per cfg2 batch at 128 B/clk,
+// and its two 32 KB raw stages kept only 64 KB of gathers in flight per SM (loaders alone: 69 us).  Here the STS and
+// the MMA's A reads are gone (144 KB per k-block) and the 64 KB of smem they occupied became two more raw stages
+// (128 KB in flight).
 //
 // Warps (24):  0-7 epilogue | 8-15 converters | 16-19 loaders | 20 MMA issuer (+ TMEM alloc) | 21 W producer |
 //              22-23 idle register donors.  Registers (pool 768 x 80): 120 | 72 | 56 | 40 | 40 | 24
@@ -14,8 +24,6 @@
 //                2 W stages {W_hi, W_lo} K-major SWIZZLE_128B (64 KB) | gamma'/beta'/attn | LN exchange | mbarriers
 // TMEM (512 columns): 2 accumulators [128 lanes x 128 fp32] | 4 A stages {hi: 32 columns, lo: 32 columns},
 //                one 32-bit column = two consecutive k of one context row (lane)
-
-#include <cstdlib>
 
 #include "c2v_tc_epilogue.cuh"
 
@@ -58,6 +66,92 @@ struct TmCfg {
     static_assert(SMEM_BYTES <= 232448, "shared memory budget");
 };
 
+// K1e pads every sub-vector and the encode size to 128 -- or to 256 in its wide configuration -- so it serves the
+// reference's default 100/100/100 (main.py:56-58) and BASELINE.json's 256/256/256 as well:
+// terminal_embed == path_embed = E, E % 4 == 0; (E <= 128 and encode_size in {100, 128}) or (E <= 256 and encode_size
+// == 256).  Row offsets are 32-bit inside the kernels: tables up to 4 GB.
+static bool tm_wide(int E, int H) { return H > TmCfg<false>::HP || E > TmCfg<false>::EP; }
+bool tcgen05_shape_ok(const c2v_dims *d)
+{
+    const int E = d->terminal_embed, H = d->encode;
+    if (d->path_embed != E || E < 4 || (E & 3)) return false;
+    const bool narrow = E <= 128 && (H == 100 || H == 128), wide = E <= 256 && H == 256;
+    if (!narrow && !wide) return false;
+    const long long row_bytes = (long long)E * 4;
+    return d->terminal_count * row_bytes < (1ll << 32) && d->path_count * row_bytes < (1ll << 32);
+}
+
+// ------------------------------------------------------------------------------------
+// weight preparation: W [H, 3E] fp32 -> 3*NQ k-block images {hi tile, lo tile} of [HP n x 64 k] fp16 in the exact
+// shared-memory layout (K-major SWIZZLE_128B), scaled by 2^k; EP = HP = 128 (NQ = 2) or 256 (NQ = 4).  Sub-vector sv
+// (start / path / end) owns k-blocks NQ*sv .. NQ*sv + NQ-1; k >= E and n >= H are zero padding.
+// ------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(1024)
+split_w_kernel(const float *__restrict__ W, uint8_t *__restrict__ img, float *__restrict__ hdr, int E, int H, int EP, int HP)
+{
+    // Several CTAs (the image is rebuilt every training step: one CTA took 22 us at 128/128/128 and 87 us at 256/256/256).
+    // Every CTA finds max |W| over the whole matrix itself (<= 768 KB, L2 hits after the first CTA): no second launch, no
+    // atomics, no pre-zeroed word.  Then one item = 4 consecutive k of one row n of the PADDED [HP][3 EP] matrix (zeros
+    // beyond E / H), i.e. 8 contiguous bytes of the hi tile and of the lo tile: every byte of the image is written once.
+    constexpr int KB = TmCfg<false>::KB;
+    __shared__ float red[32];
+    const int tid = threadIdx.x;
+    const int D = 3 * E, NQ = EP / KB;
+    const int tile_bytes = HP * KB * 2, kb_bytes = 2 * tile_bytes;
+    const bool vec = (reinterpret_cast<uintptr_t>(W) & 15) == 0;       // E % 4 == 0 on this path: rows are 16-B multiples
+    float mx = 0.0f;
+    if (vec) {
+        const float4 *W4 = reinterpret_cast<const float4 *>(W);
+        for (int i = tid; i < H * D / 4; i += 1024) {
+            const float4 v = W4[i];
+            mx = fmaxf(mx, fmaxf(fmaxf(fabsf(v.x), fabsf(v.y)), fmaxf(fabsf(v.z), fabsf(v.w))));
+        }
+    } else {
+        for (int i = tid; i < H * D; i += 1024) mx = fmaxf(mx, fabsf(W[i]));
+    }
+    mx = warp_max(mx);
+    if ((tid & 31) == 0) red[tid >> 5] = mx;
+    __syncthreads();
+    mx = red[0];
+    for (int i = 1; i < 32; ++i) mx = fmaxf(mx, red[i]);
+    // largest power of two with max|W| * scale < 2^14 (fp16 max is 65504)
+    float scale = 1.0f;
+    if (mx > 0.0f && mx < 3.0e38f) {
+        int e;
+        frexpf(mx, &e);                       // mx = f * 2^e, f in [0.5, 1)
+        int k = 14 - e;
+        k = k > 60 ? 60 : (k < -60 ? -60 : k);
+        scale = ldexpf(1.0f, k);
+    }
+    if (blockIdx.x == 0 && tid == 0) { hdr[0] = 1.0f / scale; hdr[1] = scale; }
+    const int per_row = 3 * EP / 4;
+    for (int g = blockIdx.x * 1024 + tid; g < HP * per_row; g += gridDim.x * 1024) {
+        const int n = g / per_row, kp = (g % per_row) * 4;
+        const int sv = kp / EP, e = kp % EP;
+        float4 w = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (n < H && e < E) {
+            const float *src = W + (size_t)n * D + sv * E + e;
+            w = vec ? *reinterpret_cast<const float4 *>(src) : make_float4(src[0], src[1], src[2], src[3]);
+        }
+        w.x *= scale; w.y *= scale; w.z *= scale; w.w *= scale;
+        const __half2 h01 = __floats2half2_rn(w.x, w.y), h23 = __floats2half2_rn(w.z, w.w);
+        const float2 f01 = __half22float2(h01), f23 = __half22float2(h23);
+        const __half2 l01 = __floats2half2_rn(w.x - f01.x, w.y - f01.y), l23 = __floats2half2_rn(w.z - f23.x, w.w - f23.y);
+        const int kb = NQ * sv + e / KB, kk = e % KB;
+        uint8_t *dst = img + (size_t)kb * kb_bytes + sw128_offset(n, kk);
+        *reinterpret_cast<uint2 *>(dst) = make_uint2(pack_h2(h01), pack_h2(h23));
+        *reinterpret_cast<uint2 *>(dst + tile_bytes) = make_uint2(pack_h2(l01), pack_h2(l23));
+    }
+}
+
+int launch_split_w_tcgen05(const c2v_dims *d, const float *W, EncodeWorkspace &ws, cudaStream_t st)
+{
+    const int P = tm_wide(d->terminal_embed, d->encode) ? 256 : 128;
+    split_w_kernel<<<P == 256 ? 24 : 12, 1024, 0, st>>>(W, reinterpret_cast<uint8_t *>(ws.w_hi), ws.prep_hdr, d->terminal_embed, d->encode, P, P);
+    C2V_LAUNCH_OK("split_w_kernel");
+    return C2V_OK;
+}
+
 __device__ __forceinline__ void tm_cp_async_cg16(uint32_t dst, const void *src) {
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
 }
@@ -88,17 +182,6 @@ __device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint32_t (&r)[8])
 }
 __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
-// -DTM_INSTRUMENT: CTA 0 accumulates the cycles each role spends in each of its barrier waits and writes them to
-// status[4 + slot] (read back by scripts/time_encode.py): who waits for whom, without a profiler.
-#ifdef TM_INSTRUMENT
-#define TM_WAIT(bar, parity, slot) do { const long long _t0 = clock64(); mbar_wait(bar, parity, status); \
-                                        tm_acc[slot] += clock64() - _t0; } while (0)
-#define TM_REPORT(slot) do { if (blockIdx.x == 0 && lane == 0) status[4 + (slot)] = tm_acc[slot]; } while (0)
-#else
-#define TM_WAIT(bar, parity, slot) mbar_wait(bar, parity, status)
-#define TM_REPORT(slot) do { } while (0)
-#endif
-
 // FULL_E: terminal_embed = path_embed = EP (no padding chunks); HV = encode_size (100, 128 or 256).
 template <bool DROPOUT, bool FULL_E, int HV>
 __global__ void __launch_bounds__(TmCfg<(HV > 128)>::THREADS, 1)
@@ -106,12 +189,6 @@ encode_tm_kernel(const EncodeArgs a)
 {
     constexpr bool WIDE = HV > 128;
     using tm = TmCfg<WIDE>;
-#ifdef TM_INSTRUMENT
-    long long tm_acc[12] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
-    const long long tm_t_start = clock64();
-    unsigned long long tm_g_start;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(tm_g_start));
-#endif
     extern __shared__ unsigned char smem_raw[];
     const uint32_t raw = smem_u32(smem_raw);
     const uint32_t base = (raw + 1023u) & ~1023u;
@@ -187,10 +264,10 @@ encode_tm_kernel(const EncodeArgs a)
             const int st = it & (tm::RAW_STAGES - 1);
             const uint32_t phase = (uint32_t)(it / tm::RAW_STAGES) & 1u;
             const uint32_t rawb = base + tm::SMEM_RAW_OFF + st * tm::RAW_BYTES;
-            TM_WAIT(bar_rfull + 8 * st, phase, 1);                 // gathered fp32 rows have landed
+            mbar_wait(bar_rfull + 8 * st, phase, status);          // gathered fp32 rows have landed
             float4 v[8];
 #pragma unroll
-            for (int c = 0; c < 8; ++c) v[c] = C2V_EXPT(a.flags, 128) ? make_float4(0.f, 0.f, 0.f, 0.f) : tm_lds_v4(rawb + ld_off[c]);
+            for (int c = 0; c < 8; ++c) v[c] = tm_lds_v4(rawb + ld_off[c]);
             // the asm volatile loads above complete in order before this arrive: the raw stage can be
             // refilled by the next gather while this warp converts out of registers
             __syncwarp();
@@ -213,20 +290,17 @@ encode_tm_kernel(const EncodeArgs a)
                     lo[2 * cc + 1] = pack_h2(__floats2half2_rn(x.z - f23.x, x.w - f23.y));
                 }
                 if (g == 0) {
-                    TM_WAIT(bar_aempty + 8 * as, aphase ^ 1u, 2);          // MMAs of the previous use retired
+                    mbar_wait(bar_aempty + 8 * as, aphase ^ 1u, status);   // MMAs of the previous use retired
                     tc_fence_after();
                 }
-                if (!C2V_EXPT(a.flags, 32)) {      // (timing experiment: skip the TMEM stores)
-                    tmem_st8(t_st + g * 8, hi);
-                    tmem_st8(t_st + tm::KB / 2 + g * 8, lo);
-                }
+                tmem_st8(t_st + g * 8, hi);
+                tmem_st8(t_st + tm::KB / 2 + g * 8, lo);
             }
             tmem_st_wait();
             tc_fence_before();
             __syncwarp();
             if (lane == 0) mbar_arrive(bar_afull + 8 * as);
         }
-        if (warp == tm::CONV_WARP0) { TM_REPORT(1); TM_REPORT(2); }
     } else if (warp < tm::MISC_WARP0) {
         // =============================== LOADERS (cp.async) ===============================
         asm volatile("setmaxnreg.dec.sync.aligned.u32 56;");
@@ -280,21 +354,17 @@ encode_tm_kernel(const EncodeArgs a)
                     const int st = it & (tm::RAW_STAGES - 1);
                     const uint32_t phase = (uint32_t)(it / tm::RAW_STAGES) & 1u;
                     const uint32_t dst = base + tm::SMEM_RAW_OFF + st * tm::RAW_BYTES + dst_lane;
-                    TM_WAIT(bar_rempty + 8 * st, phase ^ 1u, 0);
+                    mbar_wait(bar_rempty + 8 * st, phase ^ 1u, status);
 #pragma unroll
                     for (int j = 0; j < tm::CPA_PER_ITEM; ++j) {
                         const uint32_t chunk = (uint32_t)(h * tm::RAW_ROW_BYTES) + qoff[j & 3];   // byte offset in the row
-                        if (FULL_E) {
-                            if (!C2V_EXPT(a.flags, 64)) tm_cp_async_cg16(dst + j * 2 * tm::RAW_ROW_BYTES, tab + (o[j] + chunk));
-                        } else if (chunk < row_bytes) {     // chunk positions at or beyond the embedding size are never
+                        if (FULL_E || chunk < row_bytes)    // chunk positions at or beyond the embedding size are never
                             tm_cp_async_cg16(dst + j * 2 * tm::RAW_ROW_BYTES, tab + (o[j] + chunk));   // written: zero since start
-                        }
                     }
                     tm_cp_async_mbar_arrive_noinc(bar_rfull + 8 * st);
                 }
             }
         }
-        if (warp == tm::LOAD_WARP0) TM_REPORT(0);
     } else if (warp >= tm::MISC_WARP0 + 2) {
         asm volatile("setmaxnreg.dec.sync.aligned.u32 24;");
     } else {
@@ -304,20 +374,21 @@ encode_tm_kernel(const EncodeArgs a)
             // The whole warp runs the loop converged and one elected lane issues: inside an `if (lane == 0)` region
             // ptxas wraps every UTCHMMA in an ELECT / BRA.U.ANY loop and rebuilds the descriptors through R2UR
             // (~25 instructions per MMA); the issuer thread was then the slowest stage of the pipeline
-            // (TM_INSTRUMENT: it waited only 15 % of the time while converters and loaders waited ~50 %).
+            // (cycle counters around the barrier waits: it waited only 15 % of the time while converters and loaders
+            // waited ~50 %).
             const uint64_t wdesc0 = umma_desc(base + tm::SMEM_W_OFF);       // stage 0, W_hi, k-step 0
             const uint32_t ta0 = tmem_base + (uint32_t)tm::A_COL0;
             int it = 0;
             for (int tl = 0; tl < my_tiles; ++tl) {
                 const int acc = WIDE ? 0 : (tl & 1);
                 const uint32_t acc_phase = (uint32_t)(tl / tm::ACC_STAGES) & 1u;
-                TM_WAIT(bar_tempty + 8 * acc, acc_phase ^ 1u, 5);
+                mbar_wait(bar_tempty + 8 * acc, acc_phase ^ 1u, status);
                 const uint32_t d_tmem = tmem_base + (uint32_t)(acc * tm::HP);
 #pragma unroll 1
                 for (int kb = 0; kb < tm::NKB; ++kb, ++it) {
                     const int as = it & (tm::A_STAGES - 1), ws = it & 1;
-                    TM_WAIT(bar_afull + 8 * as, (uint32_t)(it / tm::A_STAGES) & 1u, 3);
-                    TM_WAIT(bar_wfull + 8 * ws, (uint32_t)(it >> 1) & 1u, 4);
+                    mbar_wait(bar_afull + 8 * as, (uint32_t)(it / tm::A_STAGES) & 1u, status);
+                    mbar_wait(bar_wfull + 8 * ws, (uint32_t)(it >> 1) & 1u, status);
                     tc_fence_after();
                     if (elect_one()) {
                         const uint64_t w_hi0 = wdesc0 + (uint64_t)(ws * (tm::W_KB_BYTES >> 4));
@@ -339,7 +410,6 @@ encode_tm_kernel(const EncodeArgs a)
                     __syncwarp();
                 }
             }
-            TM_REPORT(3); TM_REPORT(4); TM_REPORT(5);
         } else if (warp == tm::MISC_WARP0 + 1) {
             // =============================== W PRODUCER ===============================
             if (lane == 0) {
@@ -347,29 +417,17 @@ encode_tm_kernel(const EncodeArgs a)
                 int kb = 0;
                 for (int it = 0; it < n_items; ++it) {
                     const int ws = it & 1;
-                    TM_WAIT(bar_wempty + 8 * ws, ((uint32_t)(it >> 1) & 1u) ^ 1u, 6);
+                    mbar_wait(bar_wempty + 8 * ws, ((uint32_t)(it >> 1) & 1u) ^ 1u, status);
                     mbar_arrive_expect_tx(bar_wfull + 8 * ws, tm::W_KB_BYTES);
                     bulk_copy_g2s(base + tm::SMEM_W_OFF + ws * tm::W_KB_BYTES, img + (size_t)kb * tm::W_KB_BYTES,
                                   tm::W_KB_BYTES, bar_wfull + 8 * ws);
                     if (++kb == tm::NKB) kb = 0;
                 }
-                TM_REPORT(6);
             }
             __syncwarp();
         }
     }
 
-#ifdef TM_INSTRUMENT
-    if (tid == 0) {                                   // epilogue warp 0 leaves last-ish
-        unsigned long long g_end;
-        asm volatile("mov.u64 %0, %globaltimer;" : "=l"(g_end));
-        if (blockIdx.x == 0) { status[4 + 11] = clock64() - tm_t_start; status[18] = (long long)(g_end - tm_g_start); }
-        atomicMin((unsigned long long *)&status[16], tm_g_start);      // host presets [16] = max, [20] = max
-        atomicMax((unsigned long long *)&status[17], g_end);
-        atomicMax((unsigned long long *)&status[19], g_end - tm_g_start);
-        atomicMin((unsigned long long *)&status[20], g_end - tm_g_start);
-    }
-#endif
     tc_fence_before();
     __syncthreads();
     if (warp == tm::MISC_WARP0) {
@@ -385,13 +443,10 @@ static int launch_tm(void (*kern)(const EncodeArgs), const EncodeArgs &a, cudaSt
     int dev = 0, sms = 0;
     C2V_CUDA_OK(cudaGetDevice(&dev));
     C2V_CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    EncodeArgs b = a;
-    const char *dbg = getenv("C2V_DEBUG_FLAGS");      // timing experiments (-DC2V_EXPERIMENTS builds only)
-    if (dbg) b.flags |= atoi(dbg);
     C2V_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
     int grid = a.n_tiles < sms ? a.n_tiles : sms;
     if (grid < 1) grid = 1;
-    C2V_CUDA_OK(launch_pdl(kern, dim3((unsigned)grid), dim3(C::THREADS), (size_t)C::SMEM_BYTES, st, b));
+    C2V_CUDA_OK(launch_pdl(kern, dim3((unsigned)grid), dim3(C::THREADS), (size_t)C::SMEM_BYTES, st, a));
     C2V_COUNT_LAUNCH();
     return C2V_OK;
 }

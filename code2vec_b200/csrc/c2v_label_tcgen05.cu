@@ -11,8 +11,6 @@
 // stores with the bias added.  Output-write bound (B*C*4 bytes).
 #include <cuda_fp16.h>
 
-#include <cstdlib>
-
 #include <cstring>
 
 #include "c2v_common.cuh"
@@ -191,7 +189,7 @@ label_gemm_v2_kernel(const uint8_t *__restrict__ imgA, const uint8_t *__restrict
                      const float *__restrict__ bias, const float *__restrict__ hdr, float *__restrict__ out,
                      int M, long long N, int nkb, int n_mt, long long n_nt, long long n_tiles,
                      unsigned long long *__restrict__ keys, unsigned *__restrict__ ticket,
-                     long long *__restrict__ argmax, float *__restrict__ maxval, int dbg, const LtLoss ls, const int per_m)
+                     long long *__restrict__ argmax, float *__restrict__ maxval, const LtLoss ls, const int per_m)
 {
     extern __shared__ unsigned char smem_raw[];
     const uint32_t raw = lt_smem_u32(smem_raw);
@@ -383,7 +381,7 @@ label_gemm_v2_kernel(const uint8_t *__restrict__ imgA, const uint8_t *__restrict
                     }
                 }
             }
-            if (want_arg && lane < n_rows && n_cols > 0 && !C2V_EXPT(dbg, 2)) {
+            if (want_arg && lane < n_rows && n_cols > 0) {
                 float m = -INFINITY;
                 if (n_cols == 32) {
 #pragma unroll
@@ -402,7 +400,7 @@ label_gemm_v2_kernel(const uint8_t *__restrict__ imgA, const uint8_t *__restrict
                 }
             }
             if (out == nullptr) { __syncwarp(); continue; }   // loss-only mode: the logits are never written
-            if (!vec_ok && !C2V_EXPT(dbg, 7)) {
+            if (!vec_ok) {
                 // Rows that are only 4-byte aligned (label_count % 4 != 0, e.g. top11's 195,299): the four column-quarter
                 // warps of a row band stage the whole [32 rows x 128 columns] band, then every warp writes 8 rows of it in
                 // segments that start on 128-byte boundaries of GLOBAL memory (5 store instructions per row instead of 4;
@@ -415,19 +413,17 @@ label_gemm_v2_kernel(const uint8_t *__restrict__ imgA, const uint8_t *__restrict
                 asm volatile("bar.sync %0, 128;" ::"r"(1 + q) : "memory");
                 const long long base_col = nt * lt::TN;
                 const int tile_cols = (int)(N - base_col < lt::TN ? N - base_col : lt::TN);
-                if (!C2V_EXPT(dbg, 1)) {
 #pragma unroll 1
-                    for (int rr = cq * 8; rr < cq * 8 + 8; ++rr) {
-                        const long long grow = (long long)mt * lt::TM + q * 32 + rr;
-                        if (grow >= M) break;
-                        float *grow_p = out + (size_t)grow * N + base_col;
-                        const int a = (int)(((size_t)grow * N + base_col) & 31);        // floats past a 128-byte boundary
-                        const float *sp = band + rr * lt2::BAND_LD;
+                for (int rr = cq * 8; rr < cq * 8 + 8; ++rr) {
+                    const long long grow = (long long)mt * lt::TM + q * 32 + rr;
+                    if (grow >= M) break;
+                    float *grow_p = out + (size_t)grow * N + base_col;
+                    const int a = (int)(((size_t)grow * N + base_col) & 31);        // floats past a 128-byte boundary
+                    const float *sp = band + rr * lt2::BAND_LD;
 #pragma unroll
-                        for (int sg = 0; sg < 5; ++sg) {
-                            const int col = sg * 32 - a + lane;
-                            if (col >= 0 && col < tile_cols) grow_p[col] = sp[col];
-                        }
+                    for (int sg = 0; sg < 5; ++sg) {
+                        const int col = sg * 32 - a + lane;
+                        if (col >= 0 && col < tile_cols) grow_p[col] = sp[col];
                     }
                 }
                 asm volatile("bar.sync %0, 128;" ::"r"(1 + q) : "memory");     // the band is restaged by the next tile
@@ -438,12 +434,7 @@ label_gemm_v2_kernel(const uint8_t *__restrict__ imgA, const uint8_t *__restrict
             for (int j = 0; j < 32; j += 4)
                 *reinterpret_cast<float4 *>(stg + lane * lt2::STG_LD + j) = make_float4(v[j], v[j + 1], v[j + 2], v[j + 3]);
             __syncwarp();
-            if (C2V_EXPT(dbg, 4)) {          // timing experiment: same bytes, but every warp block as one contiguous 4 KB run
-                float *gp = out + ((size_t)(t_lo + i) * 16 + warp) * 1024 + lane * 4;
-#pragma unroll
-                for (int it = 0; it < 8; ++it)
-                    *reinterpret_cast<float4 *>(gp + it * 128) = *reinterpret_cast<const float4 *>(stg + (it * 4 + (lane >> 3)) * lt2::STG_LD + (lane & 7) * 4);
-            } else if (n_rows > 0 && n_cols > 0 && !C2V_EXPT(dbg, 1)) {
+            if (n_rows > 0 && n_cols > 0) {
                 if (vec_ok && n_cols == 32) {
                     const int rr0 = lane >> 3, c4 = (lane & 7) * 4;          // 4 rows x 128 B per store instruction
                     float *gp = out + (size_t)(row0 + rr0) * N + col0 + c4;
@@ -698,18 +689,13 @@ int launch_label_tcgen05_ex(const c2v_dims *d, const float *cv, int B, const flo
     C2V_CUDA_OK(cudaFuncSetAttribute(label_gemm_v2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, lt2::SMEM_BYTES));
     const long long n_tiles = (long long)mt * (long long)nt;
     const int grid = (int)(n_tiles < sms ? n_tiles : sms);
-    // tile order (see lt_range): lanes when that keeps >= 95 % of the CTAs busy, else groups; C2V_LABEL_ORDER=groups|lanes forces one
+    // tile order (see lt_range): lanes when that keeps >= 95 % of the CTAs busy, else groups
     int per_m = (mt <= (size_t)grid) ? grid / (int)mt : 0;
     if (per_m > 0 && (long long)per_m * (long long)mt * 100 < 95ll * grid) per_m = 0;
-    if (const char *ord = getenv("C2V_LABEL_ORDER")) {
-        if (!strcmp(ord, "groups")) per_m = 0;
-        else if (!strcmp(ord, "lanes") && mt <= (size_t)grid) per_m = grid / (int)mt;
-    }
     C2V_CUDA_OK(launch_pdl(label_gemm_v2_kernel, dim3((unsigned)grid), dim3(lt2::THREADS), (size_t)lt2::SMEM_BYTES, st,
                            (const uint8_t *)imgA, (const uint8_t *)imgB, bias, (const float *)hdr, out, B, C, nkb, (int)mt,
                            (long long)nt, n_tiles, fused_arg ? keys : (unsigned long long *)nullptr, ticket,
-                           fused_arg ? argmax : (long long *)nullptr, fused_arg ? maxval : (float *)nullptr,
-                           getenv("C2V_K2_FLAGS") ? atoi(getenv("C2V_K2_FLAGS")) : 0, ls, per_m));
+                           fused_arg ? argmax : (long long *)nullptr, fused_arg ? maxval : (float *)nullptr, ls, per_m));
     C2V_LAUNCH_OK("label_gemm_v2_kernel");
     if (want_loss) {
         loss_partials_reduce_kernel<<<dim3((unsigned)(Mpad / 32), LT_PSPLIT), 256, 0, st>>>(part, (int)(nt * 4), Mpad, part2);

@@ -1,4 +1,4 @@
-// c2v_tc_epilogue.cuh -- the epilogue role shared by the tcgen05 encode kernels (8 warps):
+// c2v_tc_epilogue.cuh -- the epilogue role of the tcgen05 encode kernel (K1e, c2v_encode_tm.cu; 8 warps):
 // TMEM -> registers, LayerNorm (model.py:55-56), tanh (:57), dropout (:60-61), score and NINF
 // masking (:64, :92-93), per-warp online-softmax partials of the weighted sum (:68-69, :96).
 #pragma once
@@ -31,13 +31,13 @@ __device__ __forceinline__ void tce_fill_vectors(const EncodeArgs &a, float *s_v
 // One tile of one epilogue thread: row `row` of the tile, columns [hf * HC, hf * HC + HC) of the accumulator.
 // The NS slices of a row are equally wide (HC = 64 at encode_size 128, 52 at 100), so all epilogue warps run the same
 // code for the same time; columns >= a.H (only in the last 4-column group of the last slice) are padding: their
-// accumulators are exactly 0 (zero rows of the W image), gamma' = beta' = attn = 0 makes their tanh output 0, `vlast`
-// (0 or 1) removes them from the variance, and they are not written anywhere.
+// accumulators are exactly 0 (zero rows of the W image), so they add nothing to the LayerNorm sums,
+// gamma' = beta' = attn = 0 makes their tanh output 0, and they are not written anywhere.
 template <bool DROPOUT, int NS, int HC>
 __device__ __forceinline__ void tce_tile_body(const EncodeArgs &a, const float *s_vec, float *my_x, const float *qx,
                                               float (&x)[(HC + 31) / 32 * 32], int q, int hf, int lane, long long vrow0,
                                               long long row, bool in_range, long long st_idx, float inv_scale,
-                                              float inv_h, float vlast, int n_valid)
+                                              float inv_h, int n_valid)
 {
     namespace tc = tce;
     static_assert(HC % 4 == 0 && HC >= 4, "columns per slice");
@@ -51,7 +51,6 @@ __device__ __forceinline__ void tce_tile_body(const EncodeArgs &a, const float *
         for (int s = 0; s < NS; ++s) t += qx[(s * 3 + slot) * 32];
         return t;
     };
-#ifndef TCE_TWOPASS_LN
     // LayerNorm (model.py:55-56), one pass: sum and sum of squares together (one exchange between the slices instead of
     // two); padding columns are exactly 0 and drop out of both.  var = E[x^2] - mean^2 in fp32: relative error
     // ~2^-24 (1 + mean^2 / var), far inside the 1e-4 budget for the row statistics of c . W^T.
@@ -67,31 +66,6 @@ __device__ __forceinline__ void tce_tile_body(const EncodeArgs &a, const float *
     named_bar_sync(1 + q, 32 * NS);
     const float mean = xsum(0) * inv_h;
     const float var = fmaxf(fmaf(-mean, mean, xsum(1) * inv_h), 0.0f) * inv_scale * inv_scale;
-    (void)vlast;
-#else
-    // LayerNorm (model.py:55-56), two-pass; x is scale * (c . W^T); slices exchanged via smem
-    float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
-#pragma unroll
-    for (int c = 0; c < HC; c += 4) { s0 += x[c]; s1 += x[c + 1]; s2 += x[c + 2]; s3 += x[c + 3]; }
-    float part = (s0 + s1) + (s2 + s3);
-    my_x[0] = part;
-    named_bar_sync(1 + q, 32 * NS);
-    const float mean = xsum(0) * inv_h;
-    s0 = s1 = s2 = s3 = 0.f;
-#pragma unroll
-    for (int c = 0; c < HC - 4; c += 4) {
-        const float d0 = x[c] - mean, d1 = x[c + 1] - mean, d2 = x[c + 2] - mean, d3 = x[c + 3] - mean;
-        s0 = fmaf(d0, d0, s0); s1 = fmaf(d1, d1, s1); s2 = fmaf(d2, d2, s2); s3 = fmaf(d3, d3, s3);
-    }
-    {
-        const float d0 = x[HC - 4] - mean, d1 = x[HC - 3] - mean, d2 = x[HC - 2] - mean, d3 = x[HC - 1] - mean;
-        s0 = fmaf(d0 * vlast, d0, s0); s1 = fmaf(d1 * vlast, d1, s1); s2 = fmaf(d2 * vlast, d2, s2); s3 = fmaf(d3 * vlast, d3, s3);
-    }
-    part = (s0 + s1) + (s2 + s3);
-    my_x[32] = part;
-    named_bar_sync(1 + q, 32 * NS);
-    const float var = xsum(1) * inv_h * inv_scale * inv_scale;
-#endif
     const float nrm = inv_scale / sqrtf(var + C2V_LN_EPS);
     const float shift = -mean * nrm;
     // tanh (model.py:57), dropout (model.py:60-61), score h.a (model.py:92-93)
@@ -173,7 +147,6 @@ __device__ __forceinline__ void tce_epilogue_loop(const EncodeArgs &a, float *s_
         static_assert(NS * HC <= tc::H && NS * HC - HV <= 4, "padding stays inside the last 4-column group of the last slice");
         static_assert(HC % 32 == 0 || HC % 32 == 16 + 4 || HC % 32 == 16 || HC % 32 == 4, "TMEM load shapes: x32, x16, x4");
         const int n_valid = (HV - hf * HC) < HC ? (HV - hf * HC) : HC;   // valid columns of this slice
-        const float vlast = n_valid == HC ? 1.0f : 0.0f;
         const float inv_scale = a.ws.prep_hdr[0];
         float *my_x = s_xch + ((q * NS + hf) * 3) * 32 + lane;          // [3][32] per (quarter, slice)
         const float *qx = s_xch + (q * NS * 3) * 32 + lane;             // slice s, slot k at qx[(s*3+k)*32]
@@ -198,7 +171,6 @@ __device__ __forceinline__ void tce_epilogue_loop(const EncodeArgs &a, float *s_
             tc_fence_before();
             __syncwarp();
             if (lane == 0) mbar_arrive(bar_tempty + 8 * acc);           // accumulator is free again
-            if (C2V_EXPT(a.flags, 16)) continue;        // timing experiment: producer side alone (results are wrong)
             if (a.stash_x && in_range) {       // training forward: keep x = c . W^T for the backward (no recompute)
                 float4 *dst = reinterpret_cast<float4 *>(a.stash_x + (size_t)row * a.H + hf * HC);
 #pragma unroll
@@ -207,7 +179,7 @@ __device__ __forceinline__ void tce_epilogue_loop(const EncodeArgs &a, float *s_
             }
 
             tce_tile_body<DROPOUT, NS, HC>(a, s_vec, my_x, qx, x, q, hf, lane, vrow0, row, in_range, st_idx,
-                                           inv_scale, 1.0f / (float)HV, vlast, n_valid);
+                                           inv_scale, 1.0f / (float)HV, n_valid);
         }
 }
 
@@ -252,7 +224,6 @@ __device__ __forceinline__ void tce_epilogue_loop_wide(const EncodeArgs &a, floa
         mbar_wait(bar_tfull, (uint32_t)tl & 1u, status);
         tc_fence_after();
         float x[CH];
-#ifndef TCE_TWOPASS_LN
         // pass 1: sum and sum of squares together (model.py:55-56; see tce_tile_body): one walk over the accumulator less
         float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f, q0 = 0.f, q1 = 0.f, q2 = 0.f, q3 = 0.f;
 #pragma unroll 1
@@ -275,39 +246,6 @@ __device__ __forceinline__ void tce_epilogue_loop_wide(const EncodeArgs &a, floa
         named_bar_sync(1 + q, 32 * NS);
         const float mean = xsum(0) * inv_h;
         const float var = fmaxf(fmaf(-mean, mean, xsum(1) * inv_h), 0.0f) * inv_scale * inv_scale;
-#else
-        // pass 1: mean (model.py:55-56)
-        float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
-#pragma unroll 1
-        for (int ch = 0; ch < NCH; ++ch) {
-            load_chunk(ch, x);
-            if (a.stash_x && in_range) {
-                float4 *dst = reinterpret_cast<float4 *>(a.stash_x + (size_t)row * a.H + hf * HS + ch * CH);
-#pragma unroll
-                for (int c = 0; c < CH; c += 4)
-                    dst[c / 4] = make_float4(x[c] * inv_scale, x[c + 1] * inv_scale, x[c + 2] * inv_scale, x[c + 3] * inv_scale);
-            }
-#pragma unroll
-            for (int c = 0; c < CH; c += 4) { s0 += x[c]; s1 += x[c + 1]; s2 += x[c + 2]; s3 += x[c + 3]; }
-        }
-        my_x[0] = (s0 + s1) + (s2 + s3);
-        named_bar_sync(1 + q, 32 * NS);
-        const float mean = xsum(0) * inv_h;
-        // pass 2: variance
-        s0 = s1 = s2 = s3 = 0.f;
-#pragma unroll 1
-        for (int ch = 0; ch < NCH; ++ch) {
-            load_chunk(ch, x);
-#pragma unroll
-            for (int c = 0; c < CH; c += 4) {
-                const float d0 = x[c] - mean, d1 = x[c + 1] - mean, d2 = x[c + 2] - mean, d3 = x[c + 3] - mean;
-                s0 = fmaf(d0, d0, s0); s1 = fmaf(d1, d1, s1); s2 = fmaf(d2, d2, s2); s3 = fmaf(d3, d3, s3);
-            }
-        }
-        my_x[32] = (s0 + s1) + (s2 + s3);
-        named_bar_sync(1 + q, 32 * NS);
-        const float var = xsum(1) * inv_h * inv_scale * inv_scale;
-#endif
         const float nrm = inv_scale / sqrtf(var + C2V_LN_EPS);
         const float shift = -mean * nrm;
         // pass 3: tanh (model.py:57), dropout (:60-61), score h.a (:92-93); h goes back into the accumulator

@@ -5,10 +5,6 @@
 
 #include "c2v_common.cuh"
 
-#ifndef C2V_SPIN_NS
-#define C2V_SPIN_NS 64
-#endif
-
 namespace c2v {
 
 // ------------------------------------------------------------------------------------
@@ -31,28 +27,17 @@ __device__ __forceinline__ void mbar_arrive_expect_tx(uint32_t bar, uint32_t byt
 // Measured alternatives (cfg2, K1e): try_wait with a suspend-time hint of 1 or 20 us: 82.6-83.1 us (the hardware
 // wake-up is slower than a poll); nanosleep 500: 74.1 us; nanosleep 64: 72.9 us  -> wake-up latency matters more than
 // the issue slots the polls take.
-#ifndef C2V_WAIT_HINT_NS
-#define C2V_WAIT_HINT_NS 0
-#endif
+constexpr unsigned C2V_SPIN_NS = 64;
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity, long long *status) {
     uint32_t ok = 0;
     long long t0 = 0;
     for (uint32_t spins = 0;; ++spins) {
-#if C2V_WAIT_HINT_NS > 0
-        asm volatile("{\n\t.reg .pred p;\n\t"
-                     "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\t"
-                     "selp.u32 %0, 1, 0, p;\n\t}"
-                     : "=r"(ok) : "r"(bar), "r"(parity), "r"((uint32_t)C2V_WAIT_HINT_NS) : "memory");
-#else
         asm volatile("{\n\t.reg .pred p;\n\t"
                      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
                      "selp.u32 %0, 1, 0, p;\n\t}"
                      : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-#endif
         if (ok) break;
-#if C2V_SPIN_NS > 0
         __nanosleep(C2V_SPIN_NS);
-#endif
 #ifndef C2V_NO_WATCHDOG                               // (compute-sanitizer slows kernels 100x: build the variant without it)
         if ((spins & 0x3ff) == 0x3ff) {
             const long long now = clock64();

@@ -15,8 +15,6 @@ There is no CPU path: parameters and inputs must live on a CUDA (B200) device.
 """
 import math
 
-import os
-
 import torch
 import torch.nn as nn
 import torch.nn.functional as F
@@ -38,7 +36,7 @@ class _EncodeFn(torch.autograd.Function):
         params = CF.make_params(emb_t, emb_p, W, ln_g, ln_b, attn)
         # when a gradient will be asked for, keep x = c . W^T (105 MB per 1024 x 200 batch at encode_size 128) so that
         # the backward neither re-gathers the embedding rows nor redoes the input_linear GEMM
-        stash = any(ctx.needs_input_grad[:6]) and os.environ.get("C2V_NO_STASH", "0") != "1"
+        stash = any(ctx.needs_input_grad[:6])
         res = CF.encode_forward(dims, params, starts, paths, ends, drop_p, training, seed, algo,
                                 cache=cache, weight=W, stash=stash)
         cv, att = res[0], res[1]

@@ -1,8 +1,6 @@
-"""Kernel-only timing of the fused encode kernel variants (CUDA events through the c2v_profile hook) + parity vs FFMA.
+"""Kernel-only timing of the fused encode kernel K1e (CUDA events through the c2v_profile hook) + parity vs FFMA.
 
-    python scripts/time_encode.py [variant[:flags] ...]      e.g.  tm cpa tm:16 tm:48
-variant = value of C2V_ENCODE_KERNEL (tm = default K1e, cpa = K1d, ldg = K1b), flags = C2V_DEBUG_FLAGS (timing
-experiments; results are wrong with flags != 0 so parity is only checked at flags 0).
+    python scripts/time_encode.py
 """
 import ctypes
 import os
@@ -30,36 +28,24 @@ D = 2 * w["Et"] + w["Ep"]
 alg_bytes = B * L * (24 + 4 * D) + B * (4 * w["H"] + 4 * L)
 ref = CF.encode_forward(dims, params, s[:B], pth[:B], e[:B], algo=_lib.ALGO_FFMA)
 cache = CF.PrepCache()
-for spec in (sys.argv[1:] or ["tm"]):
-    var, _, fl = spec.partition(":")
-    os.environ["C2V_ENCODE_KERNEL"] = var
-    os.environ["C2V_DEBUG_FLAGS"] = fl or "0"
-    W = p["input_linear.weight"]
-    if not fl or fl == "0":
-        a = CF.encode_forward(dims, params, s[:B], pth[:B], e[:B], algo=_lib.ALGO_TCGEN05)
-        err = max((a[0] - ref[0]).abs().max().item(), (a[1] - ref[1]).abs().max().item())
-    else:
-        err = float("nan")
-    for i in range(20):
-        o = (i % nb) * B
-        CF.encode_forward(dims, params, s[o:o + B], pth[o:o + B], e[o:o + B], algo=_lib.ALGO_TCGEN05, cache=cache, weight=W)
-    torch.cuda.synchronize()
-    lib.c2v_profile_enable(1)
-    n = 400
-    for i in range(n):
-        o = (i % nb) * B
-        CF.encode_forward(dims, params, s[o:o + B], pth[o:o + B], e[o:o + B], algo=_lib.ALGO_TCGEN05, cache=cache, weight=W)
-    torch.cuda.synchronize()
-    ms = ctypes.c_double(0); cnt = ctypes.c_int64(0)
-    lib.c2v_profile_read(ctypes.byref(ms), ctypes.byref(cnt))
-    lib.c2v_profile_enable(0)
-    us = ms.value / cnt.value * 1e3
-    if os.environ.get("TM_INSTRUMENT"):
-        st = cache.buf[:256].view(torch.int64).cpu().tolist()
-        print(f"   globaltimer ns: kernel span={st[17] - st[16]}  CTA0={st[18]}  CTA max={st[19]}  CTA min={st[20]}  (CTA0 cycles/ns = {st[15] / max(st[18], 1):.3f})")
-        names = ["ld:rempty", "cv:rfull", "cv:aempty", "mma:afull", "mma:wfull", "mma:tempty", "w:wempty"]
-        print("   wait cycles (CTA 0): " + "  ".join(f"{n}={st[4 + i]}" for i, n in enumerate(names)) + f"  total={st[15]}")
-    print(f"{wl} {var} flags={fl or 0}: {us:.2f} us/launch  {alg_bytes / us / 1e3:.0f} GB/s  frac={alg_bytes / us / 1e3 / peak:.3f}  max|err vs ffma|={err:.2e}", flush=True)
+W = p["input_linear.weight"]
+a = CF.encode_forward(dims, params, s[:B], pth[:B], e[:B], algo=_lib.ALGO_TCGEN05)
+err = max((a[0] - ref[0]).abs().max().item(), (a[1] - ref[1]).abs().max().item())
+for i in range(20):
+    o = (i % nb) * B
+    CF.encode_forward(dims, params, s[o:o + B], pth[o:o + B], e[o:o + B], algo=_lib.ALGO_TCGEN05, cache=cache, weight=W)
+torch.cuda.synchronize()
+lib.c2v_profile_enable(1)
+n = 400
+for i in range(n):
+    o = (i % nb) * B
+    CF.encode_forward(dims, params, s[o:o + B], pth[o:o + B], e[o:o + B], algo=_lib.ALGO_TCGEN05, cache=cache, weight=W)
+torch.cuda.synchronize()
+ms = ctypes.c_double(0); cnt = ctypes.c_int64(0)
+lib.c2v_profile_read(ctypes.byref(ms), ctypes.byref(cnt))
+lib.c2v_profile_enable(0)
+us = ms.value / cnt.value * 1e3
+print(f"{wl} encode_tm_kernel: {us:.2f} us/launch  {alg_bytes / us / 1e3:.0f} GB/s  frac={alg_bytes / us / 1e3 / peak:.3f}  max|err vs ffma|={err:.2e}", flush=True)
 if os.environ.get("TIME_FFMA"):
     for i in range(3):
         CF.encode_forward(dims, params, s[:B], pth[:B], e[:B], algo=_lib.ALGO_FFMA, cache=cache, weight=p["input_linear.weight"])

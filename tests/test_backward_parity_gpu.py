@@ -180,11 +180,11 @@ def test_tensor_core_dw_matches_the_cuda_core_gemm_at_many_tiles_per_cta(E, H, B
     d_cv = cuda((1e-6 * rng.standard_normal((B, H))).astype(np.float32))
     shapes = {"terminal_embedding": (T, E), "path_embedding": (P, E), "input_linear": (H, 3 * E), "ln_weight": (H,),
               "ln_bias": (H,), "attention": (H,)}
-    os.environ["C2V_BACKWARD_DW"] = "ffma"; os.environ["C2V_BACKWARD_DC"] = "ffma"
+    os.environ["C2V_BACKWARD"] = "ffma"
     try:
         g_ffma = CF.encode_backward(dims, params, s, pp, e, cv, att, d_cv, None, shapes)
     finally:
-        del os.environ["C2V_BACKWARD_DW"]; del os.environ["C2V_BACKWARD_DC"]
+        del os.environ["C2V_BACKWARD"]
     g_tc = CF.encode_backward(dims, params, s, pp, e, cv, att, d_cv, None, shapes)
     a, b = g_tc["input_linear"].cpu().numpy(), g_ffma["input_linear"].cpu().numpy()
     assert 1e-8 < np.abs(b).max() < 1e-3
