@@ -31,9 +31,9 @@ __device__ __forceinline__ void tce_fill_vectors(const EncodeArgs &a, float *s_v
 // One tile of one epilogue thread: row `row` of the tile, columns [hf * HC, hf * HC + HC) of the accumulator.
 // The NS slices of a row are equally wide (HC = 64 at encode_size 128, 52 at 100), so all epilogue warps run the same
 // code for the same time; columns >= a.H (only in the last 4-column group of the last slice) are padding: their
-// accumulators are exactly 0 (zero rows of the W image), so they add nothing to the LayerNorm sums,
-// gamma' = beta' = attn = 0 makes their tanh output 0, and they are not written anywhere.
-template <bool DROPOUT, int NS, int HC>
+// accumulators are exactly 0 (zero rows of the W image), so they add nothing to the LayerNorm sums and are left out
+// of the squared deviations, gamma' = beta' = attn = 0 makes their tanh output 0, and they are not written anywhere.
+template <bool DROPOUT, int NS, int HC, int HV>
 __device__ __forceinline__ void tce_tile_body(const EncodeArgs &a, const float *s_vec, float *my_x, const float *qx,
                                               float (&x)[(HC + 31) / 32 * 32], int q, int hf, int lane, long long vrow0,
                                               long long row, bool in_range, long long st_idx, float inv_scale,
@@ -51,21 +51,39 @@ __device__ __forceinline__ void tce_tile_body(const EncodeArgs &a, const float *
         for (int s = 0; s < NS; ++s) t += qx[(s * 3 + slot) * 32];
         return t;
     };
-    // LayerNorm (model.py:55-56), one pass: sum and sum of squares together (one exchange between the slices instead of
-    // two); padding columns are exactly 0 and drop out of both.  var = E[x^2] - mean^2 in fp32: relative error
-    // ~2^-24 (1 + mean^2 / var), far inside the 1e-4 budget for the row statistics of c . W^T.
-    float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f, q0 = 0.f, q1 = 0.f, q2 = 0.f, q3 = 0.f;
+    // LayerNorm (model.py:55-56) moments, two-pass within the slice: the slice's sum over its n_valid columns, then
+    // M2_s = sum (x - m_s)^2 about the slice mean m_s from the same registers.  The slices exchange (sum_s, M2_s) once and
+    // combine them with Chan's formula M2 = sum M2_s + sum n_s (m_s - mean)^2.  Unlike E[x^2] - mean^2 this does not
+    // cancel when a row's |mean| / std is large (a component shared by all rows of input_linear.weight, which LayerNorm
+    // removes and the loss never sees): the variance keeps fp32 relative accuracy there.  Padding columns (zero
+    // accumulators) are masked out of M2_s and n_s.
+    float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
 #pragma unroll
     for (int c = 0; c < HC; c += 4) {
         s0 += x[c]; s1 += x[c + 1]; s2 += x[c + 2]; s3 += x[c + 3];
-        q0 = fmaf(x[c], x[c], q0); q1 = fmaf(x[c + 1], x[c + 1], q1); q2 = fmaf(x[c + 2], x[c + 2], q2); q3 = fmaf(x[c + 3], x[c + 3], q3);
     }
     float part = (s0 + s1) + (s2 + s3);
+    const float m_s = part / (float)n_valid;
+    s0 = s1 = s2 = s3 = 0.f;
+#pragma unroll
+    for (int c = 0; c < HC; c += 4) {
+        if (c + 4 < HC || c < n_valid) {                          // only the last 4-column group can be padding
+            const float d0 = x[c] - m_s, d1 = x[c + 1] - m_s, d2 = x[c + 2] - m_s, d3 = x[c + 3] - m_s;
+            s0 = fmaf(d0, d0, s0); s1 = fmaf(d1, d1, s1); s2 = fmaf(d2, d2, s2); s3 = fmaf(d3, d3, s3);
+        }
+    }
     my_x[0] = part;
-    my_x[32] = (q0 + q1) + (q2 + q3);
+    my_x[32] = (s0 + s1) + (s2 + s3);
     named_bar_sync(1 + q, 32 * NS);
     const float mean = xsum(0) * inv_h;
-    const float var = fmaxf(fmaf(-mean, mean, xsum(1) * inv_h), 0.0f) * inv_scale * inv_scale;
+    float m2 = 0.0f;
+#pragma unroll
+    for (int s = 0; s < NS; ++s) {                               // slice order: the same bits in every slice
+        const float n_s = (float)(HV - s * HC < HC ? HV - s * HC : HC);
+        const float d = qx[(s * 3) * 32] / n_s - mean;
+        m2 += fmaf(n_s * d, d, qx[(s * 3 + 1) * 32]);
+    }
+    const float var = m2 * inv_h * inv_scale * inv_scale;
     const float nrm = inv_scale / sqrtf(var + C2V_LN_EPS);
     const float shift = -mean * nrm;
     // tanh (model.py:57), dropout (model.py:60-61), score h.a (model.py:92-93)
@@ -178,17 +196,17 @@ __device__ __forceinline__ void tce_epilogue_loop(const EncodeArgs &a, float *s_
                     if (c < n_valid) dst[c / 4] = make_float4(x[c] * inv_scale, x[c + 1] * inv_scale, x[c + 2] * inv_scale, x[c + 3] * inv_scale);
             }
 
-            tce_tile_body<DROPOUT, NS, HC>(a, s_vec, my_x, qx, x, q, hf, lane, vrow0, row, in_range, st_idx,
-                                           inv_scale, 1.0f / (float)HV, n_valid);
+            tce_tile_body<DROPOUT, NS, HC, HV>(a, s_vec, my_x, qx, x, q, hf, lane, vrow0, row, in_range, st_idx,
+                                               inv_scale, 1.0f / (float)HV, n_valid);
         }
 }
 
 // ------------------------------------------------------------------------------------------------------------------
 // encode_size 256 (BASELINE.json configs[3]): the accumulator is [128 rows x 256 columns] and there is only one of it
 // (TMEM: 256 accumulator + 256 A-stage columns), so the epilogue cannot keep a row in registers.  Warp (q, hf) owns rows
-// 32q.. and columns [128 hf, 128 hf + 128), walks them in 64-column chunks and goes over the accumulator four times:
-// sums -> mean | squared deviations -> variance | LayerNorm + tanh (+ dropout) + score, tanh output written BACK into
-// the accumulator (tcgen05.st) | softmax partials of the weighted sum from that output.  The MMAs of the next tile wait
+// 32q.. and columns [128 hf, 128 hf + 128), walks them in 64-column chunks and goes over the accumulator three times:
+// LayerNorm moments | LayerNorm + tanh (+ dropout) + score, tanh output written BACK into the accumulator
+// (tcgen05.st) | softmax partials of the weighted sum from that output.  The MMAs of the next tile wait
 // for the last pass (bar_tempty), the loaders and converters keep running (4 A stages in TMEM).
 // ------------------------------------------------------------------------------------------------------------------
 template <bool DROPOUT>
@@ -224,8 +242,10 @@ __device__ __forceinline__ void tce_epilogue_loop_wide(const EncodeArgs &a, floa
         mbar_wait(bar_tfull, (uint32_t)tl & 1u, status);
         tc_fence_after();
         float x[CH];
-        // pass 1: sum and sum of squares together (model.py:55-56; see tce_tile_body): one walk over the accumulator less
-        float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f, q0 = 0.f, q1 = 0.f, q2 = 0.f, q3 = 0.f;
+        // pass 1: LayerNorm moments (model.py:55-56), two-pass within each 64-column chunk held in registers (sum, then
+        // squared deviations about the chunk mean), chunks and then slices combined with Chan's formula as in
+        // tce_tile_body: no cancellation at large |mean| / std, and still one walk over the accumulator
+        float ssum = 0.f, m2 = 0.f;
 #pragma unroll 1
         for (int ch = 0; ch < NCH; ++ch) {
             load_chunk(ch, x);
@@ -235,20 +255,40 @@ __device__ __forceinline__ void tce_epilogue_loop_wide(const EncodeArgs &a, floa
                 for (int c = 0; c < CH; c += 4)
                     dst[c / 4] = make_float4(x[c] * inv_scale, x[c + 1] * inv_scale, x[c + 2] * inv_scale, x[c + 3] * inv_scale);
             }
+            float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
 #pragma unroll
             for (int c = 0; c < CH; c += 4) {
                 s0 += x[c]; s1 += x[c + 1]; s2 += x[c + 2]; s3 += x[c + 3];
-                q0 = fmaf(x[c], x[c], q0); q1 = fmaf(x[c + 1], x[c + 1], q1); q2 = fmaf(x[c + 2], x[c + 2], q2); q3 = fmaf(x[c + 3], x[c + 3], q3);
             }
+            const float csum = (s0 + s1) + (s2 + s3);
+            const float m_c = csum * (1.0f / CH);
+            s0 = s1 = s2 = s3 = 0.f;
+#pragma unroll
+            for (int c = 0; c < CH; c += 4) {
+                const float d0 = x[c] - m_c, d1 = x[c + 1] - m_c, d2 = x[c + 2] - m_c, d3 = x[c + 3] - m_c;
+                s0 = fmaf(d0, d0, s0); s1 = fmaf(d1, d1, s1); s2 = fmaf(d2, d2, s2); s3 = fmaf(d3, d3, s3);
+            }
+            m2 += (s0 + s1) + (s2 + s3);
+            if (ch > 0) {                       // merge with the chunks before: + n_a n_b / (n_a + n_b) (m_c - m_a)^2
+                const float d = m_c - ssum / (float)(ch * CH);
+                m2 = fmaf((float)(ch * CH) / (float)(ch + 1) * d, d, m2);
+            }
+            ssum += csum;
         }
-        my_x[0] = (s0 + s1) + (s2 + s3);
-        my_x[32] = (q0 + q1) + (q2 + q3);
+        my_x[0] = ssum;
+        my_x[32] = m2;
         named_bar_sync(1 + q, 32 * NS);
         const float mean = xsum(0) * inv_h;
-        const float var = fmaxf(fmaf(-mean, mean, xsum(1) * inv_h), 0.0f) * inv_scale * inv_scale;
+        m2 = 0.0f;
+#pragma unroll
+        for (int s = 0; s < NS; ++s) {                           // slice order: the same bits in every slice
+            const float d = qx[(s * 3) * 32] * (1.0f / HS) - mean;
+            m2 += fmaf(HS * d, d, qx[(s * 3 + 1) * 32]);
+        }
+        const float var = m2 * inv_h * inv_scale * inv_scale;
         const float nrm = inv_scale / sqrtf(var + C2V_LN_EPS);
         const float shift = -mean * nrm;
-        // pass 3: tanh (model.py:57), dropout (:60-61), score h.a (:92-93); h goes back into the accumulator
+        // pass 2: tanh (model.py:57), dropout (:60-61), score h.a (:92-93); h goes back into the accumulator
         float u0 = 0.f, u1 = 0.f;
 #pragma unroll 1
         for (int ch = 0; ch < NCH; ++ch) {
@@ -283,7 +323,7 @@ __device__ __forceinline__ void tce_epilogue_loop_wide(const EncodeArgs &a, floa
         const float u = xsum(2);
         const float z = (in_range && st_idx > 0) ? u : C2V_NINF;     // model.py:93
         if (hf == 0 && in_range) a.attention[row] = z;
-        // pass 4: per-(warp, bag) online-softmax partials of the weighted sum
+        // pass 3: per-(warp, bag) online-softmax partials of the weighted sum
         if (vrow0 < a.N) {
             const long long vt = vrow0 / tc::VROWS;
             long long last = vrow0 + tc::VROWS - 1; if (last > a.N - 1) last = a.N - 1;

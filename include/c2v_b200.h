@@ -139,7 +139,15 @@ int c2v_encode_supports_tcgen05(const c2v_dims *d);
  *   starts/paths/ends : int64 [B, L] device
  *   code_vector [B, H], attention [B, L] : fp32 device, overwritten
  * Workspace holds the split weights, the per-(tile,bag) softmax partials and a
- * status word; contents are needed by c2v_encode_backward for the same batch. */
+ * status word; contents are needed by c2v_encode_backward for the same batch.
+ * Operand range of the tensor-core path (algo TCGEN05 / AUTO; the FFMA path is plain fp32): every fp32 operand
+ * of a GEMM is split into fp16 hi + lo.  input_linear.weight, W_out and the gradients are first scaled by a power
+ * of two from their max |value|; the gathered embeddings (here and in the dW backward) and the code vectors (label
+ * GEMM and its backward) are split as they are.  So those must satisfy |value| < 65504 (fp16 overflow; not
+ * checked), and they keep full fp32-level accuracy only above about 2^-8 in magnitude: below 2^-14 the lo half is
+ * an fp16 subnormal, which caps each element's absolute precision at about 2^-25.  LayerNorm makes the forward
+ * insensitive to that (tested at embedding std 2^-8 .. 2^8); the dW backward's relative error grows as about
+ * 2^-25 / std(embedding). */
 size_t c2v_encode_workspace_bytes(const c2v_dims *d, int32_t B, int32_t L);
 int c2v_encode_forward(const c2v_dims *d, const c2v_params *p,
                        const int64_t *starts, const int64_t *paths, const int64_t *ends,
